@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # our sm_100a path
     python bench.py --impl reference --gpus N --steps K ...   # the UNMODIFIED reference (baseline/_ref) on host CPU cores
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+    python bench.py ... --dump-outputs DIR                    # + the last timed step's outputs as DIR/<name>.npy
 
 Default workload = BASELINE.json configs[2], the configuration the metric is quoted on: Conformer-L (conformer_large.yaml:
 12L/512d/8h RoPEMHA encoder, 6L decoder, vocab 5000, n_fft=512), random init, batch = 32 x 10 s @ 16 kHz synthetic per GPU,
@@ -114,6 +115,23 @@ def synth_batch(B, seconds, seed):
     import torch
     g = torch.Generator().manual_seed(seed)
     return torch.randn(B, int(SAMPLE_RATE * seconds), generator=g), torch.ones(B)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: {name: tensor} -> out_dir/<name>.npy, floating tensors as float32 and integer ones (token ids) as
+    float64, so that the outputs of two builds on the same seeded inputs can be compared array by array."""
+    import numpy as np
+    arrs = {k: v.detach().cpu().float().numpy() if v.is_floating_point() else v.detach().cpu().double().numpy()
+            for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrs.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes (limit {DUMP_LIMIT_BYTES})")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrs.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 # =============================================================================================== reference arm
@@ -300,7 +318,13 @@ def main():
     ap.add_argument("--group", type=int, default=16, help="max batches whose decode is coalesced into one greedy loop")
     ap.add_argument("--decode-steps", type=int, default=48, help="diagnostic: override the pinned 48 decode steps")
     ap.add_argument("--fuse-dec-ln", type=int, default=1)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the outputs of the last timed step "
+                    "as DIR/<name>.npy (float32 / float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.ref_threads = args.ref_threads or None
     global DECODE_STEPS
     DECODE_STEPS = args.decode_steps
@@ -546,6 +570,8 @@ def run_greedy32(args):
                 "gpu_launches": int(launches), "gpu_launches_per_step": int(launches) // max(K, 1), "clocks": clocks,
                 "roofline": roof, "cpu_baseline": cpu_base, "gpu_eager_reference": gpu_eager}
         print(json.dumps(line))
+        if args.dump_outputs:  # the token ids of the last batch of the device-resident leg's last group call
+            dump_outputs(args.dump_outputs, {"token_ids": preds[(n_calls - 1) % NL][sizes[-1] - 1]})
     if world > 1:
         dist.destroy_process_group()
 
@@ -660,10 +686,12 @@ def run_other(args):
         dec = asr.mods["decoder"]
         T = asr.engine().num_frames(L)[1]
         hyp_buf = torch.full((B, DECODE_STEPS), -1, dtype=torch.int32, device=dev)
+        last_hyps = []
 
         def step(host):
             w, l_ = (wav_host, lens_host) if host else (wav_dev, lens_dev)
             words, hyps = asr.transcribe_batch(w, l_)  # public API: encode (fused pipeline) + beam search + host replay
+            last_hyps[:] = hyps
             if world > 1:
                 hyp_buf.fill_(-1)
                 for b, h in enumerate(hyps):
@@ -720,6 +748,15 @@ def run_other(args):
                              "note": "whole step vs the encoder FLOP roofline (SURVEY 8d); the decode loop of the beam configs "
                                      "is weight-bandwidth / latency bound, see DESIGN.md"}}
         print(json.dumps(line))
+        if args.dump_outputs:  # the last timed step: encoder states, or the best hypotheses padded with -1
+            if small:
+                out = {"encoder_out": enc_out}
+            else:
+                ids = torch.full((B, max(map(len, last_hyps), default=0)), -1, dtype=torch.int32)
+                for b, h in enumerate(last_hyps):
+                    ids[b, : len(h)] = torch.tensor(h, dtype=torch.int32)
+                out = {"token_ids": ids}
+            dump_outputs(args.dump_outputs, out)
     if world > 1:
         dist.destroy_process_group()
 

@@ -128,6 +128,23 @@ def test_scorer_builder_mirrors_reference_validation():
     TransformerLMScorer(language_model=lm, temperature=1.15)
 
 
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: token ids land as exact float64, activations as float32; a dump over the limit is refused."""
+    import numpy as np
+
+    import bench
+    ids = torch.tensor([[5, 4999, -1], [7, 8, 2]], dtype=torch.int32)
+    enc = torch.randn(2, 3, 4).half()
+    bench.dump_outputs(str(tmp_path / "out"), {"token_ids": ids, "encoder_out": enc})
+    a, e = np.load(tmp_path / "out" / "token_ids.npy"), np.load(tmp_path / "out" / "encoder_out.npy")
+    assert a.dtype == np.float64 and np.array_equal(a, ids.numpy())
+    assert e.dtype == np.float32 and np.array_equal(e, enc.float().numpy())
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 16)
+    with pytest.raises(SystemExit):
+        bench.dump_outputs(str(tmp_path / "big"), {"x": torch.zeros(5)})
+    assert not (tmp_path / "big").exists()
+
+
 def test_no_undefined_names_in_package():
     """Static check (the GPU-only code paths cannot run on the CPU box): every name loaded in speechbrain_b200/*.py, bench.py
     and __graft_entry__.py is defined somewhere in its module (imports, defs, assignments, arguments, comprehensions)."""
